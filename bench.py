@@ -258,6 +258,26 @@ def timed(fn, steps, warmup, dev, world):
     return float(ms) / steps
 
 
+DUMP_GAUSSIANS = 65536      # gradient rows sampled per parameter (59 floats each: 15.5 MB)
+DUMP_PIXELS = 262144        # pixels sampled over the local views (colour+depth and alpha: 5.2 MB)
+
+
+def dump_outputs(out_dir, engine):
+    """Writes what ``engine.step()`` computed in its last call as float32 ``<name>.npy``: the gradients it returns, summed
+    over the views (v_means, v_quats, v_scales, v_opac, v_sh), for a fixed seeded sample of the Gaussians, and the local
+    views' render (colors [.., 4] = RGB + depth, alphas) for a fixed seeded sample of their pixels.  The samples depend only
+    on the sizes, so two builds of the project can be compared array for array."""
+    os.makedirs(out_dir, exist_ok=True)
+    g = torch.Generator().manual_seed(0)
+    rows = torch.randperm(engine.N, generator=g)[:DUMP_GAUSSIANS].sort().values.to(engine.dev)
+    for name in ("v_means", "v_quats", "v_scales", "v_opac", "v_sh"):
+        np.save(os.path.join(out_dir, f"{name}.npy"), engine.grads[name][rows].float().cpu().numpy())
+    cols, alps = engine.render
+    pix = torch.randperm(len(cols) * H * W, generator=g)[:DUMP_PIXELS].sort().values.to(engine.dev)
+    np.save(os.path.join(out_dir, "colors.npy"), torch.stack(cols).reshape(-1, 4)[pix].cpu().numpy())
+    np.save(os.path.join(out_dir, "alphas.npy"), torch.stack(alps).reshape(-1)[pix].cpu().numpy())
+
+
 def event_ms(fn, reps, warmup=3):
     for _ in range(warmup):
         fn()
@@ -506,7 +526,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-mast3r", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the config-3 stream and config-5 legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (rank 0, sampled)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -548,6 +572,8 @@ def main():
     sampler = ClockSampler(local_rank) if rank == 0 else None
     ms_step = timed(engine.step, args.steps, args.warmup, dev, world)
     n_isect_local = engine.check_overflow()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, engine)     # before the stage-timing steps below overwrite the buffers
 
     # per-stage live timing + launch count over K more steps, eager (CUDA events on the launching stream)
     engine.use_graph = False

@@ -30,7 +30,7 @@ def rel(a, b):
 
 
 @torch.inference_mode()
-def run(cfg, H, W, tag, stride):
+def run(cfg, H, W, tag, stride, tok_stride, scale_stride):
     model = build_ref(cfg, (H, W))
     sd = synthetic.det_weights(mt.param_shapes(cfg))
     missing = model.load_state_dict(sd, strict=False)
@@ -60,17 +60,24 @@ def run(cfg, H, W, tag, stride):
         errs["h1." + k] = rel(o1[k], r1[k]); errs["h2." + k] = rel(o2[k], r2[k])
     print(f"[{tag}] oracle vs reference:", {k: f"{v:.2e}" for k, v in errs.items()})
     assert max(errs.values()) < 2e-5, errs
-    s = stride
-    gold = dict(cfg=cfg, H=H, W=W, stride=s, enc1=f1[:, ::s].clone(), dec1_last=d1[-1][:, ::s].clone(), dec2_mid=d2[6][:, ::s].clone(),
+    s, ts, c = stride, tok_stride, scale_stride
+    gold = dict(cfg=cfg, H=H, W=W, stride=s, tok_stride=ts, enc1=f1[:, ::ts].clone(), dec1_last=d1[-1][:, ::ts].clone(),
+                dec2_mid=d2[6][:, ::ts].clone(),
                 enc_absmax=float(f1.abs().max()), dec_absmax=float(d1[-1].abs().max()))
+    # each tensor's scale (max |x|) over a grid denser than the stored one: the tests' tolerance is relative to it
+    gold.update({"enc1.scale": float(f1[:, ::c].abs().max()), "dec1_last.scale": float(d1[-1][:, ::c].abs().max()),
+                 "dec2_mid.scale": float(d2[6][:, ::c].abs().max())})
     for k in ("pts3d", "conf", "desc", "desc_conf"):
         gold["h1." + k] = r1[k][:, ::s, ::s].clone(); gold["h2." + k] = r2[k][:, ::s, ::s].clone()
         gold["h1." + k + ".absmax"] = float(r1[k].abs().max())
+        gold["h1." + k + ".scale"] = float(r1[k][:, ::c, ::c].abs().max())
+        gold["h2." + k + ".scale"] = float(r2[k][:, ::c, ::c].abs().max())
     torch.save(gold, pathlib.Path(__file__).parent / f"mast3r_{tag}.pt")
     print(f"[{tag}] wrote golden; |pts3d|max={gold['h1.pts3d.absmax']:.3f} conf max={float(r1['conf'].max()):.3f}")
 
 
 if __name__ == "__main__":
-    run(mt.SMALL_CFG, 64, 48, "small", 1)
+    run(mt.SMALL_CFG, 64, 48, "small", 1, 1, 1)
     if "--full" in sys.argv:
-        run(mt.FULL_CFG, 512, 512, "full", 8)
+        # every 64th token and every 16th pixel keep the file under 1 MB; scales over every 8th
+        run(mt.FULL_CFG, 512, 512, "full", 16, 64, 8)

@@ -1,6 +1,10 @@
 """Shared helpers for the parity tests."""
+import pathlib
+
 import numpy as np
 import torch
+
+GOLDEN = pathlib.Path(__file__).parent / "golden"
 
 # North-star tolerance (BASELINE.json): "within 1e-4 relative fp32 for rendered RGB/depth, pointmaps and
 # Gaussian gradients".  Relative to the tensor's scale (max |ref|), which is how a field of values that
@@ -30,3 +34,15 @@ def assert_close(a, b, rtol=RTOL, what="", max_outlier_frac=0.0):
     frac = bad.mean()
     assert frac <= max_outlier_frac, (f"{what}: {bad.sum()} of {bad.size} elements exceed rtol={rtol} "
                                       f"(max rel err {np.abs(a64 - b64).max() / scale:.3e})")
+
+
+def golden_sample(n, k, seed=0):
+    """Fixed sample of k flat indices out of n, shared by tests/golden/make_reference_builds_golden.py and the tests that
+    read what it stored."""
+    return np.random.default_rng(seed).choice(n, size=min(k, n), replace=False)
+
+
+def reference_builds():
+    """Seeded samples of what the reference's own CUDA extensions computed on the tests' inputs (written on a B200 by
+    tests/golden/make_reference_builds_golden.py)."""
+    return np.load(GOLDEN / "reference_builds.npz")

@@ -5,7 +5,7 @@ import pytest
 import torch
 
 from oracle import ssim_ref
-from helpers import assert_close, rel_err
+from helpers import assert_close, golden_sample, reference_builds
 
 
 def test_oracle_window_matches_reference_constants():
@@ -84,24 +84,25 @@ def test_ssim_rejects_cpu_tensors(cuda):
         fused_ssim(torch.rand(1, 3, 16, 16), torch.rand(1, 3, 16, 16))
 
 
+def _sampled(t, n):
+    return t.detach().reshape(-1)[torch.from_numpy(golden_sample(t.numel(), n)).to(t.device)].cpu()
+
+
 @pytest.mark.gpu
 def test_matches_the_reference_cuda_build(cuda):
-    """oracle/_ref/fused_ssim_ref.so is the reference's OWN ssim.cu compiled for sm_100 (--use_fast_math, as its setup.py does)."""
-    from oracle import build_ref
-    try:
-        ref = build_ref.load("fused_ssim_ref")
-    except Exception as e:  # noqa: BLE001
-        pytest.skip(f"reference extension unavailable: {e}")
+    """Against the reference's OWN ssim.cu compiled for sm_100 (--use_fast_math, as its setup.py does): a seeded sample of
+    its outputs on these inputs is stored in tests/golden/reference_builds.npz."""
     from artdeco_b200.ssim import fusedssim, fusedssim_backward
+    gold = reference_builds()
+    n = len(gold["ssim_map"])
     g = torch.Generator().manual_seed(3)
     a, b = torch.rand(2, 3, 270, 480, generator=g).to(cuda), torch.rand(2, 3, 270, 480, generator=g).to(cuda)
     C1, C2 = 0.01 ** 2, 0.03 ** 2
-    mr, r1, r2, r3 = ref.fusedssim(C1, C2, a, b, True)
     mo, o1, o2, o3 = fusedssim(C1, C2, a, b, True)
-    assert_close(mo, mr, rtol=1e-5, what="ssim map vs reference build")
-    assert_close(o1, r1, rtol=1e-5, what="dm_dmu1")
+    assert_close(_sampled(mo, n), gold["ssim_map"], rtol=1e-5, what="ssim map vs reference build")
+    assert_close(_sampled(o1, n), gold["ssim_dm_dmu1"], rtol=1e-5, what="dm_dmu1")
     up = torch.rand(2, 3, 270, 480, generator=g).to(cuda)
-    assert_close(fusedssim_backward(C1, C2, a, b, up, o1, o2, o3), ref.fusedssim_backward(C1, C2, a, b, up, r1, r2, r3),
+    assert_close(_sampled(fusedssim_backward(C1, C2, a, b, up, o1, o2, o3), n), gold["ssim_grad"],
                  rtol=1e-5, what="dL/dimg1 vs reference build")
 
 
@@ -110,8 +111,11 @@ def test_matches_the_reference_cuda_build(cuda):
 def test_ssim_full_size_matches_oracle_and_reference_build(cuda, shape):
     """Full-size check as in the reference's own test (fused-ssim/tests/test.py:57-91: B=5, CH=5, 1080x1920) and at the
     BASELINE shape [1,3,1080,1920]: scalar and gradient against the conv2d formulation (the oracle; fp64 on the GPU so
-    it takes milliseconds), and map / derivative / gradient against the reference's own ssim.cu built into oracle/_ref."""
+    it takes milliseconds), and map / gradient against stored samples of the reference's own ssim.cu on these inputs."""
     from artdeco_b200.ssim import fused_ssim, fusedssim, fusedssim_backward
+    gold = reference_builds()
+    tag = {(1, 3, 1080, 1920): "baseline_1x3x1080p", (5, 5, 1080, 1920): "reference_test_5x5x1080p"}[shape]
+    gmap, ggrad = gold[f"ssim_full_{tag}_map"], gold[f"ssim_full_{tag}_grad"]
     g = torch.Generator().manual_seed(5)
     a = torch.rand(*shape, generator=g).to(cuda)
     b = torch.rand(*shape, generator=g).to(cuda)
@@ -123,15 +127,9 @@ def test_ssim_full_size_matches_oracle_and_reference_build(cuda, shape):
     out.backward()
     assert abs(float(out.detach()) - float(ref.detach())) <= 1e-5 * abs(float(ref.detach())) + 2e-7
     assert_close(a_gpu.grad, a_ref.grad, what="dL/dimg1 (full size)")
-    from oracle import build_ref
-    try:
-        rb = build_ref.load("fused_ssim_ref")
-    except Exception as e:  # noqa: BLE001
-        pytest.skip(f"reference extension unavailable (oracle half of this test passed): {e}")
     C1, C2 = 0.01 ** 2, 0.03 ** 2
-    mr, r1, r2, r3 = rb.fusedssim(C1, C2, a, b, True)
     mo, o1, o2, o3 = fusedssim(C1, C2, a, b, True)
-    assert_close(mo, mr, rtol=1e-5, what="ssim map vs reference build (full size)")
+    assert_close(_sampled(mo, len(gmap)), gmap, rtol=1e-5, what="ssim map vs reference build (full size)")
     up = torch.rand(*shape, generator=g).to(cuda)
-    assert_close(fusedssim_backward(C1, C2, a, b, up, o1, o2, o3), rb.fusedssim_backward(C1, C2, a, b, up, r1, r2, r3),
+    assert_close(_sampled(fusedssim_backward(C1, C2, a, b, up, o1, o2, o3), len(ggrad)), ggrad,
                  rtol=1e-5, what="dL/dimg1 vs reference build (full size)")
